@@ -68,7 +68,12 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the kv / join / file-path extras (1 GPU)")
     ap.add_argument("--no-parity", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the TF-IDF table of the last timed end-to-end step to DIR/*.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def dist_env():
@@ -255,6 +260,30 @@ def read_sink_lines(out_dir):
         with open(os.path.join(out_dir, fn), "rb") as f:
             lines.extend(f.read().split(b"\n"))
     return sorted(l for l in lines if l)
+
+
+DUMP_LIMIT = 64 << 20  # bytes of .npy data dump_outputs writes at most
+
+
+def dump_outputs(out_dir, dump_dir, suffix=""):
+    """The sink_tsv table a TF-IDF step wrote to `out_dir` (term, document frequency, idf), as float64 columns in term
+    order: term_hash.npy (the first 52 bits of the term's blake2b digest, exact in a float64), doc_freq.npy, idf.npy.
+    A table larger than DUMP_LIMIT is cut to a seeded sample of rows (the same rows for the same table size)."""
+    lines = read_sink_lines(out_dir)
+    cols = {"term_hash": np.empty(len(lines)), "doc_freq": np.empty(len(lines)), "idf": np.empty(len(lines))}
+    for i, l in enumerate(lines):
+        term, df, idf = l.split(b"\t")
+        cols["term_hash"][i] = int.from_bytes(hashlib.blake2b(term, digest_size=8).digest(), "little") >> 12
+        cols["doc_freq"][i] = int(df)
+        cols["idf"][i] = float(idf)
+    rows = DUMP_LIMIT // (8 * len(cols))
+    if len(lines) > rows:
+        keep = np.sort(np.random.default_rng(0).choice(len(lines), rows, replace=False))
+        cols = {k: v[keep] for k, v in cols.items()}
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, col in cols.items():
+        np.save(os.path.join(dump_dir, name + suffix + ".npy"), col)
+    return len(lines)
 
 
 def warm_page_cache(path):
@@ -653,6 +682,9 @@ def main():
         n_terms_total = int(t[0].item())
     else:
         n_terms_total = n_terms
+    if args.dump_outputs:
+        dumped = dump_outputs(d, args.dump_outputs, "" if world == 1 else "_rank%d" % rank)
+        progress("dumped the %d-row TF-IDF table of the last timed step to %s" % (dumped, args.dump_outputs))
 
     total = nbytes * world
     value_dev = total * args.steps / t_dev / MB

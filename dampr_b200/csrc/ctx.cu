@@ -671,9 +671,11 @@ int32_t dampr_textbuf_upload(dampr_ctx *ctx, dampr_textbuf *tb, uint64_t off, co
 }
 
 // ---- GPUDirect Storage ingest (cuFile), opt-in: dampr_set_option("file_cufile", 1) ---------------------------
-// libcufile is bound at run time. cuFileRead moves file bytes to device memory without the page-locked ring: by
-// DMA from the NVMe controller where the nvidia-fs driver and an O_DIRECT-capable file system are present, through
-// cuFile's own bounce buffers ("compatibility mode") elsewhere. Several host threads issue disjoint 16 MB reads.
+// libcufile is bound at run time. cuFileRead moves file bytes to device memory without the page-locked ring, by
+// DMA from the NVMe controller, where the nvidia-fs driver and an O_DIRECT-capable file system are present. Without
+// the driver the path is refused before libcufile is touched: cuFile's "compatibility mode" only copies through its
+// own bounce buffers, which the ring does too, and on B200 machines without the driver its cuFileRead blocked for
+// good. Several host threads issue disjoint 16 MB reads.
 namespace {
 
 struct CuFileApi {
@@ -690,6 +692,10 @@ CuFileApi *cufile_api() {
     static CuFileApi api;
     static std::once_flag once;
     std::call_once(once, [] {
+        if (access("/proc/driver/nvidia-fs/version", F_OK) != 0) {
+            api.why = "the nvidia-fs (GPUDirect Storage) driver is not loaded";
+            return;
+        }
         const char *names[] = {"libcufile.so.0", "libcufile.so", "/usr/local/cuda/targets/x86_64-linux/lib/libcufile.so.0"};
         for (const char *n : names) {
             api.lib = dlopen(n, RTLD_NOW);
@@ -716,13 +722,13 @@ CuFileApi *cufile_api() {
         }
         api.driver_open = true;
     });
-    return api.lib ? &api : nullptr;
+    return &api;
 }
 
 int cufile_h2d(dampr_ctx *ctx, void *dst, const char *path, size_t foff, size_t bytes) {
     CuFileApi *a = cufile_api();
-    if (!a) {
-        return set_err(ctx, DAMPR_ERR_CUDA, "cuFile is not available: %s", "dlopen / cuFileDriverOpen failed");
+    if (!a->driver_open) {
+        return set_err(ctx, DAMPR_ERR_CUDA, "cuFile is not available: %s", a->why.c_str());
     }
     // O_DIRECT first (what GPUDirect Storage wants); a file system that refuses it, or whose registration fails
     // with it, gets a second try with a plain descriptor (cuFile's compatibility mode)

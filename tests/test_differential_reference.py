@@ -1,18 +1,43 @@
-"""Differential test against the REAL reference, when it is importable (the development container has it at
-/root/reference; elsewhere the test skips): seeded random DSL pipelines run through Refefer/Dampr's own
+"""Differential test against the REAL reference: seeded random DSL pipelines run through Refefer/Dampr's own
 MTRunner and through this engine's runner (on the numpy stand-in for the device, tests/fake_device.py) must
 give the same multiset of results. This pins the DSL semantics of the host layer — stage fusion, keyed
-records, combiners, joins — to the reference itself rather than to a restatement."""
+records, combiners, joins — to the reference itself rather than to a restatement.
+
+The reference's results on the seeded inputs are stored in tests/golden/differential_reference.json.gz. To record
+them again from a checkout of the reference (after a change to a pipeline or an input):
+
+    DAMPR_REFERENCE=<checkout of Refefer/Dampr> python -m pytest tests/test_differential_reference.py
+"""
+import gzip
 import os
 import random
 import subprocess
 import sys
 import json
+import tempfile
 
 import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "dampr")), reason="reference checkout not present")
+REF = os.environ.get("DAMPR_REFERENCE")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "differential_reference.json.gz")
+
+
+def reference(case, driver, *args):
+    """The last stdout line of `python -c driver <reference checkout> *args`, parsed as JSON: the stored result for
+    `case`, or, when DAMPR_REFERENCE names a checkout, the result of running the reference now, which is stored."""
+    with gzip.open(GOLDEN, "rt") as f:
+        stored = json.load(f)
+    if not REF:
+        return stored[case]
+    env = dict(os.environ)
+    env.pop("PYTHONPATH", None)   # the reference's `dampr` package, not this repository's shim
+    p = subprocess.run([sys.executable, "-c", driver, REF] + list(args), capture_output=True, text=True, env=env,
+                       cwd=tempfile.gettempdir(), timeout=600)
+    assert p.returncode == 0, p.stderr[-2000:]
+    stored[case] = json.loads(p.stdout.strip().split("\n")[-1])
+    with open(GOLDEN, "wb") as f:
+        f.write(gzip.compress(json.dumps(stored, sort_keys=True, separators=(",", ":")).encode(), mtime=0))
+    return stored[case]
 
 
 def pipelines(seed, n_cases):
@@ -73,12 +98,7 @@ def test_random_pipelines_agree_with_the_reference(monkeypatch):
     items = [rng.randint(-50, 200) for _ in range(300)]
     srcs = pipelines(2024, 60)
     # the reference runs in its own interpreter (its `dampr` package would shadow the shim here)
-    env = dict(os.environ)
-    env.pop("PYTHONPATH", None)
-    p = subprocess.run([sys.executable, "-c", DRIVER, REF, json.dumps(items), json.dumps(srcs)], capture_output=True,
-                       text=True, env=env, cwd="/tmp", timeout=240)
-    assert p.returncode == 0, p.stderr[-2000:]
-    ref = json.loads(p.stdout.strip().split("\n")[-1])
+    ref = reference("random_pipelines", DRIVER, json.dumps(items), json.dumps(srcs))
     monkeypatch.setattr(runner_mod, "_CTX", {settings.device: FakeCtx()})
     monkeypatch.setattr(plan, "_BUFFERS", {})
     for src, exp in zip(srcs, ref):
@@ -152,12 +172,7 @@ def test_random_text_pipelines_agree_with_the_reference(path_kind, monkeypatch, 
             f.write(data)
         longest = max([len(l) + 1 for l in data.split(b"\n")] + [1]) if ci < 4 else len(data) + 1
         srcs = text_pipelines(100 + ci, 14, longest)
-        env = dict(os.environ)
-        env.pop("PYTHONPATH", None)
-        p = subprocess.run([sys.executable, "-c", TEXT_DRIVER, REF, path, json.dumps(srcs)], capture_output=True,
-                           text=True, env=env, cwd="/tmp", timeout=240)
-        assert p.returncode == 0, p.stderr[-2000:]
-        ref = json.loads(p.stdout.strip().split("\n")[-1])
+        ref = reference("text_pipelines_%d" % ci, TEXT_DRIVER, path, json.dumps(srcs))
         if path_kind == "host-map":
             monkeypatch.setattr(runner_mod, "_CTX", {settings.device: FakeCtx()})
         else:
@@ -206,12 +221,7 @@ def test_more_random_pipelines_agree_with_the_reference(monkeypatch):
         rng = random.Random(seed)
         items = [rng.randint(-50, 200) for _ in range(n_items)]
         srcs = more_pipelines(seed * 17, 40)
-        env = dict(os.environ)
-        env.pop("PYTHONPATH", None)
-        p = subprocess.run([sys.executable, "-c", DRIVER, REF, json.dumps(items), json.dumps(srcs)], capture_output=True,
-                           text=True, env=env, cwd="/tmp", timeout=240)
-        assert p.returncode == 0, p.stderr[-2000:]
-        ref = json.loads(p.stdout.strip().split("\n")[-1])
+        ref = reference("more_pipelines_%d" % seed, DRIVER, json.dumps(items), json.dumps(srcs))
         monkeypatch.setattr(runner_mod, "_CTX", {settings.device: FakeCtx()})
         monkeypatch.setattr(plan, "_BUFFERS", {})
         for src, exp in zip(srcs, ref):
@@ -250,12 +260,7 @@ def test_sinks_write_the_lines_the_reference_writes(monkeypatch, tmp_path):
         "Dampr.memory(items, partitions=4).map(lambda x: 'line %d' % x).sink(out)",
         "Dampr.memory(items, partitions=1).mean(lambda x: x % 3, lambda x: x).sink_tsv(out)",
     ]
-    env = dict(os.environ)
-    env.pop("PYTHONPATH", None)
-    p = subprocess.run([sys.executable, "-c", SINK_DRIVER, REF, json.dumps(items), json.dumps(templates), str(tmp_path)],
-                       capture_output=True, text=True, env=env, cwd="/tmp", timeout=240)
-    assert p.returncode == 0, p.stderr[-2000:]
-    ref = json.loads(p.stdout.strip().split("\n")[-1])
+    ref = reference("sinks", SINK_DRIVER, json.dumps(items), json.dumps(templates), str(tmp_path))
     monkeypatch.setattr(runner_mod, "_CTX", {settings.device: FakeCtx()})
     monkeypatch.setattr(plan, "_BUFFERS", {})
     for i, (src, exp) in enumerate(zip(templates, ref)):
@@ -290,12 +295,7 @@ def test_key_types_agree_with_the_reference(monkeypatch):
     rng = random.Random(5)
     items = [rng.randint(-50, 200) for _ in range(90)]
     srcs = key_type_pipelines()
-    env = dict(os.environ)
-    env.pop("PYTHONPATH", None)
-    p = subprocess.run([sys.executable, "-c", DRIVER, REF, json.dumps(items), json.dumps(srcs)], capture_output=True,
-                       text=True, env=env, cwd="/tmp", timeout=400)
-    assert p.returncode == 0, p.stderr[-2000:]
-    ref = json.loads(p.stdout.strip().split("\n")[-1])
+    ref = reference("key_types", DRIVER, json.dumps(items), json.dumps(srcs))
     monkeypatch.setattr(runner_mod, "_CTX", {settings.device: FakeCtx()})
     monkeypatch.setattr(plan, "_BUFFERS", {})
     for src, exp in zip(srcs, ref):
@@ -348,12 +348,7 @@ def test_inputs_outputs_and_empty_cases_agree_with_the_reference(monkeypatch, tm
      "sorted(Dampr.memory(items).filter(lambda x: False).a_group_by(lambda x: 1).sum().join(Dampr.memory(items).a_group_by(lambda x: 1).sum()).reduce(lambda l, r: 1).run())",
      "sorted(Dampr.memory(items).a_group_by(lambda x: 1).sum().join(Dampr.memory(items).filter(lambda x: False).a_group_by(lambda x: 1).sum()).left_reduce(lambda l, r: (list(l), list(r))).run())",
     ]
-    env = dict(os.environ)
-    env.pop("PYTHONPATH", None)
-    p = subprocess.run([sys.executable, "-c", EXPR_DRIVER, REF, json.dumps(items), json.dumps(srcs), jpath],
-                       capture_output=True, text=True, env=env, cwd="/tmp", timeout=400)
-    assert p.returncode == 0, p.stderr[-2000:]
-    ref = json.loads(p.stdout.strip().split("\n")[-1])
+    ref = reference("inputs_outputs_and_empty_cases", EXPR_DRIVER, json.dumps(items), json.dumps(srcs), jpath)
     monkeypatch.setattr(runner_mod, "_CTX", {settings.device: FakeCtx()})
     monkeypatch.setattr(plan, "_BUFFERS", {})
     for src, exp in zip(srcs, ref):
@@ -391,12 +386,7 @@ def test_lowered_kv_and_frame_stages_agree_with_the_reference(monkeypatch):
     for h in heads:
         for t in tails:
             srcs_ref.append("Dampr.memory(recs, partitions=3)"+h+t); srcs_ours.append("Dampr.read_input(ArrayKVInput(K, V))"+h+t)
-    env = dict(os.environ)
-    env.pop("PYTHONPATH", None)
-    p = subprocess.run([sys.executable, "-c", RECS_DRIVER, REF, json.dumps(list(zip(keys, vals))), json.dumps(srcs_ref)],
-                       capture_output=True, text=True, env=env, cwd="/tmp", timeout=600)
-    assert p.returncode == 0, p.stderr[-2000:]
-    ref = json.loads(p.stdout.strip().split("\n")[-1])
+    ref = reference("lowered_kv_and_frame_stages", RECS_DRIVER, json.dumps(list(zip(keys, vals))), json.dumps(srcs_ref))
     K, V = np.array(keys, dtype=np.int64), np.array(vals, dtype=np.int64)
     lowered = 0
     for so, exp in zip(srcs_ours, ref):
@@ -441,12 +431,7 @@ for fn in sorted(os.listdir(out)):
         lines.extend(l.rstrip("\n") for l in f)
 print(json.dumps(sorted(lines)))
 """
-    env = dict(os.environ)
-    env.pop("PYTHONPATH", None)
-    p = subprocess.run([sys.executable, "-c", driver, REF, json.dumps(list(zip(keys, vals))), ref_src, str(tmp_path / "ref")],
-                       capture_output=True, text=True, env=env, cwd="/tmp", timeout=300)
-    assert p.returncode == 0, p.stderr[-2000:]
-    exp = json.loads(p.stdout.strip().split("\n")[-1])
+    exp = reference("lowered_cross_and_sink", driver, json.dumps(list(zip(keys, vals))), ref_src, str(tmp_path / "ref"))
     monkeypatch.setattr(runner_mod, "_CTX", {settings.device: FakeCtx()})
     monkeypatch.setattr(plan, "_BUFFERS", {})
     K, V = np.array(keys, dtype=np.int64), np.array(vals, dtype=np.int64)
@@ -498,13 +483,8 @@ def test_lowered_joins_probes_and_sorts_agree_with_the_reference(monkeypatch):
      "{A}.sort_by(lambda x: -x[0])",
      "{A}.a_group_by(lambda x: x[0], lambda x: x[1]).sum().cross_right({B}.len(), lambda kv, n: (kv[0], kv[1] * n))",
     ]
-    env = dict(os.environ)
-    env.pop("PYTHONPATH", None)
-    p = subprocess.run([sys.executable, "-c", TWO_DRIVER, REF, json.dumps(list(zip(keys, vals))),
-                        json.dumps([t.format(A=A_ref, B=B_ref) for t in tmpl]), json.dumps(list(zip(k2, v2)))],
-                       capture_output=True, text=True, env=env, cwd="/tmp", timeout=600)
-    assert p.returncode == 0, p.stderr[-2000:]
-    ref = json.loads(p.stdout.strip().split("\n")[-1])
+    ref = reference("lowered_joins_probes_and_sorts", TWO_DRIVER, json.dumps(list(zip(keys, vals))),
+                    json.dumps([t.format(A=A_ref, B=B_ref) for t in tmpl]), json.dumps(list(zip(k2, v2))))
     ns = {"Dampr": Dampr, "ArrayKVInput": ArrayKVInput, "K": np.array(keys, dtype=np.int64), "V": np.array(vals, dtype=np.int64),
           "K2": np.array(k2, dtype=np.int64), "V2": np.array(v2, dtype=np.int64)}
     seen = set()
@@ -541,12 +521,7 @@ def test_directory_inputs_agree_with_the_reference(path_kind, monkeypatch, tmp_p
         f.write(gen.text(4, 80, V=50))
     longest = max(len(l) + 1 for data in files.values() for l in data.split(b"\n")) + 5
     srcs = text_pipelines(900, 12, longest)
-    env = dict(os.environ)
-    env.pop("PYTHONPATH", None)
-    p = subprocess.run([sys.executable, "-c", TEXT_DRIVER, REF, str(d), json.dumps(srcs)], capture_output=True, text=True,
-                       env=env, cwd="/tmp", timeout=300)
-    assert p.returncode == 0, p.stderr[-2000:]
-    ref = json.loads(p.stdout.strip().split("\n")[-1])
+    ref = reference("directory_inputs", TEXT_DRIVER, str(d), json.dumps(srcs))
     monkeypatch.setattr(plan, "_pinned_ring", lambda n, b: [F.FakePinned(b) for _ in range(n)])
     for src, exp in zip(srcs, ref):
         monkeypatch.setattr(runner_mod, "_CTX", {settings.device: F.FakeCtx() if path_kind == "host-map" else F.FakeTextCtx()})
@@ -585,12 +560,7 @@ def test_crlf_gzip_inputs_agree_with_the_reference(path_kind, monkeypatch, tmp_p
             ".len()",
             ".map(lambda x: x)",
         )]
-        env = dict(os.environ)
-        env.pop("PYTHONPATH", None)
-        p = subprocess.run([sys.executable, "-c", TEXT_DRIVER, REF, str(d), json.dumps(srcs)], capture_output=True, text=True,
-                           env=env, cwd="/tmp", timeout=300)
-        assert p.returncode == 0, p.stderr[-2000:]
-        ref = json.loads(p.stdout.strip().split("\n")[-1])
+        ref = reference("crlf_gzip_" + layout, TEXT_DRIVER, str(d), json.dumps(srcs))
         assert repr("hello world\r") in ref[4] if layout == "gz-only" else True
         monkeypatch.setattr(plan, "_pinned_ring", lambda n, b: [F.FakePinned(b) for _ in range(n)])
         for src, exp in zip(srcs, ref):
@@ -631,14 +601,9 @@ def test_lowered_join_idioms_agree_with_the_reference(monkeypatch):
         "{B}" + G + ".join({A}" + G + ").reduce(lambda l, r: itertools.product(l, r), many=True)",   # duplicate right keys
         "{A}" + G + ".join({B}" + G + ").reduce(lambda l, r: (sum(l), sorted(r)))",                   # not an idiom
     ]
-    env = dict(os.environ)
-    env.pop("PYTHONPATH", None)
     driver = TWO_DRIVER.replace("import sys, json", "import sys, json, itertools")
-    p = subprocess.run([sys.executable, "-c", driver, REF, json.dumps(list(zip(keys, vals))),
-                        json.dumps([t.format(A=A_ref, B=B_ref) for t in tmpl]), json.dumps(list(zip(k2, v2)))],
-                       capture_output=True, text=True, env=env, cwd="/tmp", timeout=600)
-    assert p.returncode == 0, p.stderr[-2000:]
-    ref = json.loads(p.stdout.strip().split("\n")[-1])
+    ref = reference("lowered_join_idioms", driver, json.dumps(list(zip(keys, vals))),
+                    json.dumps([t.format(A=A_ref, B=B_ref) for t in tmpl]), json.dumps(list(zip(k2, v2))))
     ns = {"Dampr": Dampr, "ArrayKVInput": ArrayKVInput, "itertools": itertools, "K": np.array(keys, dtype=np.int64),
           "V": np.array(vals, dtype=np.int64), "K2": np.array(k2, dtype=np.int64), "V2": np.array(v2, dtype=np.int64)}
     hows = []
@@ -689,13 +654,8 @@ def test_lowered_topk_unique_prefix_agree_with_the_reference(monkeypatch):
         "{A}" + S + ".map(lambda x: (x[0], x[1], x[1] / 7.0)).sink_json(__import__('tempfile').mkdtemp())",
         "{A}" + S + ".map(lambda x: x[1] * 0.5).sink_json(__import__('tempfile').mkdtemp())",
     ]
-    env = dict(os.environ)
-    env.pop("PYTHONPATH", None)
-    p = subprocess.run([sys.executable, "-c", TWO_DRIVER, REF, json.dumps(list(zip(keys, vals))),
-                        json.dumps([t.format(A=A_ref) for t in tmpl]), json.dumps([])],
-                       capture_output=True, text=True, env=env, cwd="/tmp", timeout=600)
-    assert p.returncode == 0, p.stderr[-2000:]
-    ref = json.loads(p.stdout.strip().split("\n")[-1])
+    ref = reference("lowered_topk_unique_prefix", TWO_DRIVER, json.dumps(list(zip(keys, vals))),
+                    json.dumps([t.format(A=A_ref) for t in tmpl]), json.dumps([]))
     ns = {"Dampr": Dampr, "ArrayKVInput": ArrayKVInput, "K": np.array(keys, dtype=np.int64), "V": np.array(vals, dtype=np.int64)}
     hows = []
     for t, exp in zip(tmpl, ref):
@@ -745,13 +705,8 @@ def test_chains_over_binary_kv_inputs_agree_with_the_reference(monkeypatch):
         "{A}.a_group_by(lambda x: x[0] % 5, lambda x: x[1]).reduce(min)",
         "{A}.map(lambda x: x[1] / 4.0).a_group_by(lambda x: 1).reduce(max)",
     ]
-    env = dict(os.environ)
-    env.pop("PYTHONPATH", None)
-    p = subprocess.run([sys.executable, "-c", TWO_DRIVER, REF, json.dumps(list(zip(keys, vals))),
-                        json.dumps([t.format(A=A_ref) for t in tmpl]), json.dumps([])],
-                       capture_output=True, text=True, env=env, cwd="/tmp", timeout=600)
-    assert p.returncode == 0, p.stderr[-2000:]
-    ref = json.loads(p.stdout.strip().split("\n")[-1])
+    ref = reference("chains_over_binary_kv_inputs", TWO_DRIVER, json.dumps(list(zip(keys, vals))),
+                    json.dumps([t.format(A=A_ref) for t in tmpl]), json.dumps([]))
     ns = {"Dampr": Dampr, "ArrayKVInput": ArrayKVInput, "K": np.array(keys, dtype=np.int64), "V": np.array(vals, dtype=np.int64)}
     hows = []
     for t, exp in zip(tmpl, ref):
@@ -773,11 +728,8 @@ def test_chains_over_binary_kv_inputs_agree_with_the_reference(monkeypatch):
         "{A}.map(lambda x: (x[0], x[1] * 3)).a_group_by(lambda x: x[0], lambda x: x[1]).sum()",
         "{A}.map(lambda x: x[0] % 7).count()",                      # arithmetic on such keys: host map
     ]
-    p = subprocess.run([sys.executable, "-c", TWO_DRIVER, REF, json.dumps(list(zip(big, vals))),
-                        json.dumps([t.format(A=A_ref) for t in tmpl2]), json.dumps([])],
-                       capture_output=True, text=True, env=env, cwd="/tmp", timeout=600)
-    assert p.returncode == 0, p.stderr[-2000:]
-    ref2 = json.loads(p.stdout.strip().split("\n")[-1])
+    ref2 = reference("chains_over_binary_kv_inputs_u64_keys", TWO_DRIVER, json.dumps(list(zip(big, vals))),
+                     json.dumps([t.format(A=A_ref) for t in tmpl2]), json.dumps([]))
     ns["K"], ns["V"] = np.array(big, dtype=np.uint64), np.array(vals, dtype=np.int64)
     for i, (t, exp) in enumerate(zip(tmpl2, ref2)):
         monkeypatch.setattr(runner_mod, "_CTX", {settings.device: FakeCtx()})

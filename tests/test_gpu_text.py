@@ -1,6 +1,8 @@
 """GPU parity: text tokenise+combine kernels (csrc/text.cu) vs the oracle restatement.
 
 Bit-exact: counts, line counts, the '' token, key strings."""
+import os
+
 import numpy as np
 import pytest
 
@@ -128,27 +130,29 @@ def test_tile_boundaries(ctx):
 
 
 def test_flags(ctx, text_kernel):
-    if text_kernel == 1:
-        pytest.skip("limits below are those of the v2 kernel")
     _, st = run_count(ctx, "café au lait\n".encode("utf-8"), dev.TOK_WS)
     assert st["flags"] & dev.TF_NONASCII
     _, st = run_count(ctx, b"a\r\nb\r\n", dev.TOK_WS)
     assert st["flags"] & dev.TF_CR          # str.split: scan-wide flag (token counts do not depend on it)
     _, st = run_count(ctx, b"a\r\nb\r\n", dev.TOK_NONWORD_LOWER_SET)
-    assert st["flags"] == 0 and st["fallback"] == 2   # [^\w]+ modes: the two lines go to the host, nothing else
+    if text_kernel == 1:
+        assert st["flags"] & dev.TF_CR and st["fallback"] == 0   # first generation: '\r' flags the whole scan
+    else:
+        assert st["flags"] == 0 and st["fallback"] == 2   # [^\w]+ modes: the two lines go to the host, nothing else
     long_line = b"x " * 20000 + b"\n"
     _, st = run_count(ctx, b"a\n" * 4000 + long_line + b"b\n" * 4000, dev.TOK_NONWORD_LOWER_SET)
-    assert st["flags"] & dev.TF_LONGLINE
-    # more distinct tokens in one line than the de-duplication history holds
+    assert st["flags"] & dev.TF_LONGLINE    # longer than either kernel's window
+    # more distinct tokens in one line than the de-duplication history of the v2 kernel holds
     many = b" ".join(b"w%d" % i for i in range(400)) + b"\n"
-    _, st = run_count(ctx, b"a b\n" * 10 + many + b"c\n", dev.TOK_NONWORD_LOWER_SET)
-    assert st["flags"] & dev.TF_LONGLINE
+    if text_kernel == 2:
+        _, st = run_count(ctx, b"a b\n" * 10 + many + b"c\n", dev.TOK_NONWORD_LOWER_SET)
+        assert st["flags"] & dev.TF_LONGLINE
     # both are fine for the first-generation kernel when they fit its 4 KB window
     dev.set_option("text_kernel", 1)
     try:
         check_df(ctx, b"a b\n" * 10 + many + b"c\n")
     finally:
-        dev.set_option("text_kernel", 2)
+        dev.set_option("text_kernel", text_kernel)
     # the whitespace tokeniser has no line dependence: long lines are fine there
     check_wc(ctx, b"a\n" * 4000 + long_line + b"b\n" * 4000)
 
@@ -199,9 +203,8 @@ def _bad_line_corpus(seed=3, n_lines=6000):
 def test_per_line_fallback_lists_exactly_the_bad_lines(ctx, text_kernel):
     """[^\\w]+ tokenisers: a line holding a byte the device cannot tokenise like Python (non-ASCII, '\\r' in text
     mode) contributes nothing to the table / line count / '' count and is reported with its offset and length;
-    everything else is counted as if those lines were not there."""
-    if text_kernel == 1:
-        pytest.skip("the first-generation kernel keeps scan-wide flags")
+    everything else is counted as if those lines were not there. The first-generation kernel keeps no such list: any
+    such byte (a '\\r' even where it is data) flags the whole scan for the host."""
     lines = _bad_line_corpus()
     data = b"\n".join(lines) + b"\n"
     for cr_is_data in (False, True):
@@ -226,6 +229,11 @@ def test_per_line_fallback_lists_exactly_the_bad_lines(ctx, text_kernel):
                     tab.count(tb, lo, hi, mode, cr_is_data)
                     lo = hi
                 st = tab.stats()
+                if text_kernel == 1:
+                    assert st["flags"] & dev.TF_NONASCII and st["flags"] & dev.TF_CR and st["fallback"] == 0, st
+                    tb.free()
+                    tab.free()
+                    continue
                 assert st["flags"] == 0, st
                 assert sorted(tab.fallback_lines().tolist()) == exp_fb
                 codes, counts, reps = tab.fetch()
@@ -250,8 +258,7 @@ def test_per_line_fallback_lists_exactly_the_bad_lines(ctx, text_kernel):
 
 
 def test_fallback_list_overflow_sets_the_scan_wide_flag(ctx, text_kernel):
-    if text_kernel == 1:
-        pytest.skip("v2 kernel only")
+    """v2: more bad lines than its list holds end in the scan-wide flag; the first-generation kernel sets it for any."""
     data = "é\n".encode() * 70000      # more bad lines than the list holds (and than a warp region may isolate)
     _, st = run_count(ctx, data, dev.TOK_NONWORD_LOWER_SET, verify=False)
     assert st["flags"] & dev.TF_NONASCII
@@ -259,7 +266,8 @@ def test_fallback_list_overflow_sets_the_scan_wide_flag(ctx, text_kernel):
 
 def test_upload_file_through_cufile_matches_the_ring(ctx, tmp_path):
     """The opt-in cuFile ingest (dampr_set_option("file_cufile", 1), csrc/ctx.cu): the same bytes land in the text
-    buffer as through the page-locked ring; token counts agree. Skipped where libcufile cannot be opened."""
+    buffer as through the page-locked ring; token counts agree. Skipped where cuFile is unavailable: without the
+    nvidia-fs driver the upload must fail at once, naming it."""
     data = gen.text(31, 30000, V=5000)
     p = tmp_path / "c.txt"
     p.write_bytes(data)
@@ -276,6 +284,7 @@ def test_upload_file_through_cufile_matches_the_ring(ctx, tmp_path):
         try:
             tb2.upload_file(0, str(p), 0, len(data))
         except dev.DeviceError as e:
+            assert os.path.exists("/proc/driver/nvidia-fs/version") or "nvidia-fs" in str(e), e
             if "cuFile" in str(e):
                 pytest.skip("cuFile unavailable here: %s" % e)
             raise
